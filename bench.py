@@ -479,7 +479,13 @@ def main():
     ap.add_argument("--no-job", dest="no_job", action="store_true", help="skip the whole-job (1M queries incl. set-up) leg")
     ap.add_argument("--no-legs", action="store_true",
                     help="default run only: skip the short configs[2] / configs[3] / configs[4] legs appended to the headline line")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="usearch / c4: write the hit table of the last timed step (device-resident path) as DIR/<field>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "vsg" or args.workload not in ("usearch", "c4")):
+        ap.error("--dump-outputs: the usearch and c4 workloads of --impl vsg only")
     if args.warmup < 3:
         args.warmup = 3
 
@@ -540,6 +546,27 @@ def main():
     usearch_workload(args, rank, world, local)
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, res, counts, work, max_results):
+    """What vsg_search_batch handed back in the last timed step: one float64 array per SearchResult field (query-major,
+    max_results slots per query; slots past counts[q] are as the library left them), counts and the work counters.
+    Above 64 MB in all, a fixed seeded sample of queries is kept and query_index.npy says which."""
+    os.makedirs(out_dir, exist_ok=True)
+    rows = np.ctypeslib.as_array(res).reshape(len(counts), max_results)
+    nq = len(counts)
+    per_query = 8 * (max_results * len(rows.dtype.names) + 1)
+    if nq * per_query > DUMP_LIMIT_BYTES:
+        keep = np.sort(np.random.default_rng(0).choice(nq, size=DUMP_LIMIT_BYTES // per_query - 1, replace=False))
+        np.save(os.path.join(out_dir, "query_index.npy"), keep.astype(np.float64))
+        rows, counts = rows[keep], counts[keep]
+    for name in rows.dtype.names:
+        np.save(os.path.join(out_dir, name + ".npy"), rows[name].astype(np.float64))
+    np.save(os.path.join(out_dir, "counts.npy"), counts.astype(np.float64))
+    np.save(os.path.join(out_dir, "work.npy"), np.asarray(work, dtype=np.float64))
+
+
 def usearch_workload(args, rank, world, local):
     """configs[1] (headline) / configs[3] shape: --usearch_global through vsg_search_batch"""
     leg = getattr(args, "leg", False)
@@ -596,6 +623,8 @@ def usearch_workload(args, rank, world, local):
             dist.barrier()
         torch.cuda.synchronize()
 
+    last = {}
+
     def run_steps(e2e: bool, lazy: bool = False, mask=None):
         """returns (device ms for the K timed steps, work, launches, profile, clocks).  mask = (db, index): the
         DUST leg — queries are masked on the device inside the timed region, database and index are the masked ones"""
@@ -630,6 +659,7 @@ def usearch_workload(args, rank, world, local):
                 work_tot += work
         ev1.record(stream)
         barrier()
+        last.update(res=res, counts=counts, work=work)
         ms = ev0.elapsed_time(ev1)
         clocks = sampler.summary() if sampler else {}
         prof = ctx.profile()
@@ -661,6 +691,8 @@ def usearch_workload(args, rank, world, local):
         ix.close(); db.close(); ctx.close()
         return
     ms_dev, work_dev, launches, prof, clocks, hits = run_steps(e2e=False)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last["res"], last["counts"], last["work"], max_results)
     ms_e2e, work_e2e, _, _, _, _ = run_steps(e2e=True)
     # optional mode, reported separately and NOT the headline: candidates are aligned only when the
     # accept/reject replay is about to examine them (same hit tables, tests/test_search_gpu.py); the

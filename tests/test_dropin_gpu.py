@@ -9,6 +9,7 @@ import time
 import numpy as np
 import pytest
 
+import checkers
 from vsearch_b200 import synth
 
 pytestmark = pytest.mark.gpu
@@ -20,6 +21,10 @@ FIELDS = "query+target+id+alnlen+mism+opens+raw+caln+qilo+qihi+tilo+tihi+id0+id1
 
 needs_bins = pytest.mark.skipif(not (os.path.exists(STOCK) and os.path.exists(GPU)),
                                 reason="oracle/_ref/vsearch{,_gpu} not built")
+
+
+def _lines_digest(lines):
+    return {"lines": len(lines), "sha256": checkers.digest("".join(lines))}
 
 
 def run(binary, args, threads):
@@ -76,7 +81,7 @@ def test_usearch_global_and_cluster_fast(tmp_path):
     assert len(ucs["cpu"]) > 3000 and ucs["cpu"] == ucs["gpu"]
 
 
-@pytest.mark.skipif(not os.path.exists(STOCK), reason="oracle/_ref/vsearch not built")
+@pytest.mark.skipif(not checkers.have_reference_cli(), reason="neither oracle/_ref nor tests/golden/reference")
 def test_allpairs_api_vs_reference_cli(tmp_path):
     """vsg_allpairs (rows sharded in two halves, as two GPUs would) against the stock CLI on configs[0]"""
     from vsearch_b200 import lib as vlib
@@ -84,9 +89,9 @@ def test_allpairs_api_vs_reference_cli(tmp_path):
     fa = str(tmp_path / "c1.fasta")
     synth.write_fasta(fa, reads, "r")
     uo = str(tmp_path / "cpu.userout")
-    run(STOCK, ["--allpairs_global", fa, "--id", "0.8", "--qmask", "none", "--userout", uo,
-                "--userfields", "query+target+id+alnlen+mism+raw+ids"], os.cpu_count())
-    want = sorted_lines(uo)
+    want = checkers.reference_cli(["--allpairs_global", fa, "--id", "0.8", "--qmask", "none", "--userout", uo,
+                                   "--userfields", "query+target+id+alnlen+mism+raw+ids", "--quiet"],
+                                  lambda: _lines_digest(sorted_lines(uo)), threads=os.cpu_count())
     ctx = vlib.Context(0)
     ss = ctx.seqset(reads)
     o = vlib.default_search_opts(); o.id = 0.8
@@ -96,7 +101,7 @@ def test_allpairs_api_vs_reference_cli(tmp_path):
     # userout's alnlen is the alignment length without terminal gaps (results.cpp / userfields)
     got = sorted(f"r{h['query']}\tr{h['target']}\t{h['id']:.1f}\t{h['internal_alignment_length']}\t{h['mismatches']}\t"
                  f"{h['nwscore']}\t{h['matches']}\n" for h in list(h1) + list(h2))
-    assert len(want) > 10000 and got == want
+    assert want["lines"] > 10000 and _lines_digest(got) == want
     assert int(w1[0] + w2[0]) == n * (n - 1) // 2
     # per query: id descending, then target ascending (allpairs_hit_compare)
     q = h1["query"]; same = q[1:] == q[:-1]

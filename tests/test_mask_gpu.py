@@ -1,7 +1,5 @@
 """Device DUST masking (vsg_seqset_dust) against the reference's dust() (core/mask.cpp) and, end to
 end, the default-masking search (--qmask dust --dbmask dust) against the compiled reference."""
-import ctypes as C
-
 import numpy as np
 import pytest
 
@@ -9,13 +7,7 @@ import checkers
 from vsearch_b200 import lib as vlib
 from vsearch_b200 import synth
 
-pytestmark = [pytest.mark.gpu, pytest.mark.skipif(checkers.ref() is None, reason="oracle/_ref/libvsref.so not present")]
-
-
-def ref_dust(seq: bytes) -> bytes:
-    b = C.create_string_buffer(seq)
-    checkers.ref().vsref_dust(b, C.c_int(len(seq)))
-    return b.value
+pytestmark = [pytest.mark.gpu, pytest.mark.skipif(not checkers.have_reference(), reason="neither oracle/_ref nor tests/golden/reference")]
 
 
 def low_complexity(rng, n):
@@ -45,7 +37,7 @@ def test_dust_matches_reference():
     sym = h.symbols(int(ss.lens.sum()))
     masked_total = 0
     for i, s in enumerate(seqs):
-        want = ref_dust(s)
+        want = checkers.ref_dust(s)
         o = int(ss.offs[i])
         got_lower = (sym[o:o + len(s)] & 16) != 0
         want_lower = np.array([97 <= c <= 122 for c in want], dtype=bool)

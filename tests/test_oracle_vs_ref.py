@@ -1,13 +1,13 @@
 """Pins the oracle (oracle/*.c) against the UNMODIFIED reference compiled into
-oracle/_ref/libvsref.so.  CPU only.  Skipped when oracle/_ref has not been built
-(the GPU box gets the prebuilt files; a bare checkout relies on tests/golden/)."""
+oracle/_ref/libvsref.so.  CPU only.  Without oracle/_ref the reference's answers are the ones stored
+under tests/golden/reference (checkers.reference_result)."""
 import numpy as np
 import pytest
 
 import checkers as _libs
 from vsearch_b200 import synth
 
-pytestmark = pytest.mark.skipif(_libs.ref() is None, reason="oracle/_ref/libvsref.so not built")
+pytestmark = pytest.mark.skipif(not _libs.have_reference(), reason="neither oracle/_ref nor tests/golden/reference")
 
 IUPAC = b"ACGTUacgtuNnRYSWKMBDHVryswkmbdhvXx-*."
 
@@ -111,8 +111,7 @@ def test_unique_kmers():
             for _ in range(20):
                 s = rand_seq(rng, int(rng.integers(0, 400)), b"ACGTACGTACGTacgtNnRU")
                 a = _libs.oracle_unique_kmers(s, k, ml)
-                b = _libs.ref_unique_kmers(s, k, ml)
-                assert np.array_equal(a, b)
+                assert _libs.kmers_digest(a) == _libs.ref_unique_kmers_digest(s, k, ml)
 
 
 def _family_db(rng, n_roots=12, per=8, L=300):
@@ -168,7 +167,7 @@ def test_large_wordlengths_match_reference(k):
     nonempty = 0
     for i, q in enumerate(qs):
         for m in (0, 1):
-            assert np.array_equal(_libs.oracle_unique_kmers(q, k, m), _libs.ref_unique_kmers(q, k, m)), (k, i, m)
+            assert _libs.kmers_digest(_libs.oracle_unique_kmers(q, k, m)) == _libs.ref_unique_kmers_digest(q, k, m), (k, i, m)
         s1, c1 = r.topscores(q)
         s2, c2 = o.topscores(q, opts)
         assert np.array_equal(s1, s2) and np.array_equal(c1, c2), (k, i)

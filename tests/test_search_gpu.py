@@ -188,7 +188,7 @@ def test_ranker_ties_and_thresholds_vs_oracle(ctx):
     od.close(); ix.close(); db.close(); qs.close()
 
 
-@pytest.mark.skipif(checkers.ref() is None, reason="oracle/_ref/libvsref.so not present")
+@pytest.mark.skipif(not checkers.have_reference(), reason="neither oracle/_ref nor tests/golden/reference")
 def test_search_vs_compiled_reference(ctx):
     """config-2 shape in miniature: 250-nt windows of a random 1500-nt database, 5 % mutated"""
     dbs, qss, src = synth.config2_search(n_db=400, db_len=1500, n_q=120, q_len=250, div=0.05, seed=77)
@@ -225,7 +225,7 @@ def test_search_vs_compiled_reference(ctx):
     ix.close(); db.close(); qs.close()
 
 
-@pytest.mark.skipif(checkers.ref() is None, reason="oracle/_ref/libvsref.so not present")
+@pytest.mark.skipif(not checkers.have_reference(), reason="neither oracle/_ref nor tests/golden/reference")
 @pytest.mark.parametrize("maxaccepts,ident", [(1, 0.9), (1, 0.97), (3, 0.9)])
 def test_traceback_on_demand_does_not_change_the_hit_tables(ctx, maxaccepts, ident):
     """the followers of a group are walked back only when the leader is not accepted (align_ckpt.cuh, TbGate): same rows
@@ -255,12 +255,11 @@ def test_traceback_on_demand_does_not_change_the_hit_tables(ctx, maxaccepts, ide
     ix.close(); db.close(); qs.close()
 
 
-@pytest.mark.skipif(checkers.ref() is None, reason="oracle/_ref/libvsref.so not present")
+@pytest.mark.skipif(not checkers.have_reference(), reason="neither oracle/_ref nor tests/golden/reference")
 def test_deferred_pairs_go_through_the_fallback_callback(ctx):
     """pairs the 16-bit aligner cannot take (q*d > 25e6) are resolved by the host application's
     linear-memory aligner through vsg_ctx_set_fallback — here the reference's own LinearMemoryAligner —
     and the hit table still equals the reference's"""
-    import ctypes as C
     import re
     rng = np.random.default_rng(41)
     big = synth.random_seqs(rng, 3, 5200)
@@ -274,15 +273,11 @@ def test_deferred_pairs_go_through_the_fallback_callback(ctx):
     r = checkers.RefDb(dbs, id=0.8, maxaccepts=2, maxrejects=8)
     want = r.search(qss, max_results=r.tophits)
     th = r.tophits
-    rlib = checkers.ref()
 
     def fallback(q, strand, t):
         assert strand == 0
-        out = (C.c_longlong * 5)()
-        qs_, ts_ = queries[q], dbs.seq(t)
-        buf = C.create_string_buffer(len(qs_) + len(ts_) + 8)
-        assert rlib.vsref_lma(C.c_void_p(r.h), qs_, C.c_int(len(qs_)), ts_, C.c_int(len(ts_)), out, buf, C.c_int(len(buf))) == 0
-        ops = re.findall(r"(\d*)([MID])", buf.value.decode())
+        out, cigar = r.lma(queries[q], dbs.seq(t))
+        ops = re.findall(r"(\d*)([MID])", cigar)
         f, l = ops[0], ops[-1]
         fr = int(f[0]) if f[0] else 1; lr = int(l[0]) if l[0] else 1
         return [out[0], out[1], out[2], out[3], out[4], fr if f[1] == "D" else 0, fr if f[1] == "I" else 0,
@@ -324,11 +319,10 @@ def test_long_queries_rank_vs_oracle(ctx):
     od.close(); ix.close(); db.close(); qs.close()
 
 
-@pytest.mark.skipif(checkers.ref() is None, reason="oracle/_ref/libvsref.so not present")
+@pytest.mark.skipif(not checkers.have_reference(), reason="neither oracle/_ref nor tests/golden/reference")
 def test_optional_filters_vs_compiled_reference(ctx):
     """--minqt/--maxqt/--minsl/--maxsl (pre-alignment rejects consume the reject budget) and
     --maxsubs/--maxgaps/--mincols/--maxdiffs/--leftjust/--rightjust/--query_cov/--target_cov/--maxid/--mid"""
-    import ctypes as C
     rng = np.random.default_rng(47)
     roots = synth.random_seqs(rng, 8, 320)
     seqs = []
@@ -358,8 +352,7 @@ def test_optional_filters_vs_compiled_reference(ctx):
         order = ["minqt", "maxqt", "minsl", "maxsl", "maxid", "mid", "query_cov", "target_cov", "maxsubs", "maxgaps",
                  "mincols", "maxdiffs", "leftjust", "rightjust"]
         r = checkers.RefDb(dbs, id=0.85, maxaccepts=3, maxrejects=6)
-        arr = (C.c_double * 14)(*[float(v[k]) for k in order])
-        checkers.ref().vsref_db_set_filters(C.c_void_p(r.h), arr)
+        r.set_filters([v[k] for k in order])
         want = r.search(qss, max_results=r.tophits)
         th = r.tophits
         r.close()

@@ -14,6 +14,8 @@ from vsearch_b200 import synth
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 STOCK = os.path.join(ROOT, "oracle", "_ref", "vsearch")
 needs_stock = pytest.mark.skipif(not os.path.exists(STOCK), reason="oracle/_ref/vsearch not built")
+# the small files below are stored under tests/golden/reference as the reference wrote them (checkers.reference_cli)
+needs_stock_or_stored = pytest.mark.skipif(not checkers.have_reference_cli(), reason="neither oracle/_ref nor tests/golden/reference")
 
 
 def make_db(tmp_path, n=300, seed=5):
@@ -44,8 +46,12 @@ def make_db(tmp_path, n=300, seed=5):
 
 
 def makeudb(fasta, out, *extra):
-    r = subprocess.run([STOCK, "--makeudb_usearch", fasta, "--output", out, "--quiet", *extra], capture_output=True, text=True, timeout=600)
-    assert r.returncode == 0, r.stderr[-2000:]
+    import base64
+    import gzip
+    data = checkers.reference_cli(["--makeudb_usearch", fasta, "--output", out, "--quiet", *extra],
+                                  lambda: base64.b64encode(gzip.compress(open(out, "rb").read(), 9, mtime=0)).decode(), timeout=600)
+    if not os.path.exists(STOCK):
+        open(out, "wb").write(gzip.decompress(base64.b64decode(data)))
 
 
 @needs_stock
@@ -96,7 +102,7 @@ def test_udb_file_vs_fasta_and_oracle_index(tmp_path, mode):
     u.close()
 
 
-@needs_stock
+@needs_stock_or_stored
 def test_invalid_udb_files_are_rejected(tmp_path):
     fasta, _ = make_db(tmp_path, n=40)
     udb = str(tmp_path / "db.udb")
@@ -124,7 +130,7 @@ def test_invalid_udb_files_are_rejected(tmp_path):
         vlib.Udb(str(tmp_path / "missing.udb"))
 
 
-@needs_stock
+@needs_stock_or_stored
 def test_c_example_builds_and_parses_a_udb_file(tmp_path):
     """examples/usearch_udb.c (plain C against include/vsg.h) compiles with gcc, links libvsg.so, reads a UDB file made by
     the reference and — in a container without a GPU — stops at the first device call with the library's error message

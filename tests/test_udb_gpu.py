@@ -71,8 +71,8 @@ def test_usearch_global_on_a_udb_file_equals_the_reference_cli(tmp_path, ctx, db
 
 
 def test_a_udb_whose_index_is_not_its_sequences_is_rejected(tmp_path, ctx):
-    if not os.path.exists(STOCK):
-        pytest.skip("oracle/_ref/vsearch not built")
+    if not checkers.have_reference_cli():
+        pytest.skip("neither oracle/_ref nor tests/golden/reference")
     fasta, _ = make_db(tmp_path, n=50)
     udb = str(tmp_path / "db.udb")
     makeudb(fasta, udb)
@@ -90,7 +90,7 @@ def test_a_udb_whose_index_is_not_its_sequences_is_rejected(tmp_path, ctx):
     u.close()
 
 
-@pytest.mark.skipif(checkers.ref() is None, reason="oracle/_ref/libvsref.so not present")
+@pytest.mark.skipif(not checkers.have_reference(), reason="neither oracle/_ref nor tests/golden/reference")
 @pytest.mark.parametrize("k", [11, 12, 13])
 def test_wordlength_above_10_vs_compiled_reference(ctx, k):
     """candidate lists (search_topscores) and whole searches with --wordlength 11..13: two shards' worth of targets
