@@ -94,6 +94,11 @@ int vsg_seqset_dust(vsg_ctx * ctx, vsg_seqset * s);
 /* the symbol bytes as stored in HBM (bits 0-3 = 4-bit nucleotide code, bit 4 = lower case), in the
  * order and at the offsets given to vsg_seqset_create; cap >= total sequence bytes.  For tools/tests. */
 int vsg_seqset_symbols(vsg_ctx * ctx, const vsg_seqset * s, uint8_t * out, int64_t cap);
+/* the reverse complements of sequences [q0, q0 + n) of `src` as a new set of n sequences (entry i = the reverse
+ * complement of sequence q0 + i): replaces reverse_complement (utils/reverse_complement.cpp:71-84).  Case, and so
+ * the soft mask, is kept; non-IUPAC symbols become 'N'.  E.g. the CIGAR of a strand-1 clustering record is
+ * vsg_align_pairs(revcomp set, set) of that sequence against its centroid.  Free with vsg_seqset_destroy. */
+int vsg_seqset_revcomp(vsg_ctx * ctx, const vsg_seqset * src, int64_t q0, int64_t n, vsg_seqset ** out);
 
 /* ---- batched alignment: replaces search16_qprep + search16 (core/align_simd.cpp:1406-2060)
  *      for npairs (query,target) pairs at once.  qidx[i] indexes `queries`, tidx[i] indexes
@@ -292,9 +297,19 @@ int vsg_allpairs(vsg_ctx * ctx, const vsg_seqset * set, int64_t row0, int64_t nr
  *      --uc) or the sequence number of the centroid it matched plus that alignment's statistics and identity
  *      (an "H" record; the CIGAR is one vsg_align_pairs call away).  NOTE the reference's default --maxrejects for
  *      --cluster_fast is 8, not 32 (cli.cc:4163-4172): set opts->maxrejects accordingly.  opts: id, iddef, maxaccepts, maxrejects,
- *      wordlength, minwordmatches, mask_lower, the length / abundance / post-alignment filters (target_sizes
- *      and target_labels are per sequence of `set`); plus strand only.  work (optional, 2 x int64): pairs and DP
- *      cells handed to the aligner. ---- */
+ *      wordlength, minwordmatches, mask_lower, strand_both, the length / abundance / post-alignment filters
+ *      (target_sizes and target_labels are per sequence of `set`).  work (optional, 2 x int64): pairs and DP cells
+ *      handed to the aligner, both strands counted.
+ *      strand_both (--strand both, cluster.cpp:162-189, 946-1025): each sequence is also searched as the reverse
+ *      complement of the sequence AS STORED, so its soft mask is mirrored and not computed again (unlike
+ *      vsg_search_batch with qmask_dust, which masks each strand on its own).  Each strand has its own candidate
+ *      list, counters and hit list; the best hit is taken over the plus hits, then the minus hits, ties going to plus.
+ *      results[i].strand = 1 when the sequence matched its centroid as the reverse complement: identity and
+ *      statistics are those of the reverse complement aligned to the centroid, and so is the CIGAR
+ *      (vsg_seqset_revcomp, then vsg_align_pairs).  New centroids are always indexed as stored (strand 0).  A
+ *      deferred pair reaches the fallback callback with the sequence's number in `set` and its strand.  The set is
+ *      mirrored once at setup into a device copy holding every sequence and its reverse complement (twice the
+ *      set's symbol bytes). ---- */
 typedef struct vsg_cluster_result {
   int32_t cluster;
   int32_t centroid;
@@ -316,7 +331,9 @@ int vsg_cluster_fast(vsg_ctx * ctx, const vsg_seqset * set, const vsg_search_opt
  *      to must outlive it.  vsg_cluster_session_assign handles the sequences [start, start + count) in rounds of
  *      round_size (cluster_assign_batch: the caller's --threads; cluster_assign_single: count = round_size = 1);
  *      ranges must be ascending and contiguous (cluster.hpp:104-111), results[i] belongs to sequence start + i.
- *      A session fed the whole set in one call gives vsg_cluster_fast's results. ---- */
+ *      A session fed the whole set in one call gives vsg_cluster_fast's results.  The set's contents must not change
+ *      after vsg_cluster_session_create (no vsg_seqset_dust in between): with strand_both the session reads its
+ *      queries, both strands, from the mirror it copied at create. ---- */
 typedef struct vsg_cluster_session vsg_cluster_session;
 int vsg_cluster_session_create(vsg_ctx * ctx, const vsg_seqset * set, const vsg_search_opts * opts, vsg_cluster_session ** out);
 int vsg_cluster_session_assign(vsg_cluster_session * session, int64_t start, int64_t count, int round_size,

@@ -425,7 +425,66 @@ int seqset_revcomp(vsg_ctx * c, const vsg_seqset * src, int64_t q0, int64_t n, v
   *out = guard.release();
   return VSG_OK;
 }
+
+// the query set of a --strand both clustering: 2n entries, 2i = sequence i as stored (case = its mask), 2i + 1 = its
+// reverse complement, back to back, so that the two strands of consecutive sequences form one contiguous range
+int seqset_strand_pairs(vsg_ctx * c, const vsg_seqset * src, vsg_seqset ** out)
+{
+  *out = nullptr;
+  vsg_seqset * s = new (std::nothrow) vsg_seqset();
+  if (s == nullptr) { Error::set("out of host memory"); return VSG_ENOMEM; }
+  SeqsetGuard guard{s};
+  int64_t const n = src->d.n, m = 2 * n;
+  s->device = c->device;
+  s->h_len.resize(static_cast<size_t>(m));
+  s->h_off.resize(static_cast<size_t>(m));
+  s->h_nonacgt.resize(static_cast<size_t>(m));
+  int64_t total = 0;
+  for (int64_t i = 0; i < n; i++) {
+    int32_t const l = src->h_len[static_cast<size_t>(i)];
+    for (int64_t e = 2 * i; e < 2 * i + 2; e++) {
+      s->h_len[static_cast<size_t>(e)] = l;
+      s->h_off[static_cast<size_t>(e)] = total;
+      s->h_nonacgt[static_cast<size_t>(e)] = src->h_nonacgt[static_cast<size_t>(i)];
+      total += l;
+    }
+  }
+  s->total = total;
+  int rc;
+  if ((rc = s->b_sym.reserve(static_cast<size_t>(total) + 64)) != VSG_OK ||
+      (rc = s->b_off.reserve(sizeof(int64_t) * static_cast<size_t>(m) + 8)) != VSG_OK ||
+      (rc = s->b_len.reserve(sizeof(int32_t) * static_cast<size_t>(m) + 8)) != VSG_OK) {
+    return rc;
+  }
+  s->d.sym = static_cast<uint8_t *>(s->b_sym.p);
+  s->d.off = static_cast<int64_t *>(s->b_off.p);
+  s->d.len = static_cast<int32_t *>(s->b_len.p);
+  s->d.n = m;
+  if (n > 0) {
+    VSG_CUDA_OK(cudaMemcpyAsync(s->b_off.p, s->h_off.data(), sizeof(int64_t) * m, cudaMemcpyHostToDevice, c->stream));
+    VSG_CUDA_OK(cudaMemcpyAsync(s->b_len.p, s->h_len.data(), sizeof(int32_t) * m, cudaMemcpyHostToDevice, c->stream));
+    int64_t const blocks = (n * 32 + 255) / 256;
+    strand_pairs_kernel<<<static_cast<unsigned>(blocks), 256, 0, c->stream>>>(src->d, s->d.off, static_cast<uint8_t *>(s->b_sym.p));
+    count_launch();
+    VSG_CUDA_OK(cudaGetLastError());
+    VSG_CUDA_OK(cudaStreamSynchronize(c->stream));
+  }
+  *out = guard.release();
+  return VSG_OK;
+}
 }  // namespace vsg
+
+extern "C" int vsg_seqset_revcomp(vsg_ctx * c, const vsg_seqset * src, int64_t q0, int64_t n, vsg_seqset ** out)
+{
+  if (c == nullptr || src == nullptr || out == nullptr || q0 < 0 || n < 0 || q0 + n > src->d.n) {
+    Error::set("vsg_seqset_revcomp: bad argument");
+    return VSG_EINVAL;
+  }
+  *out = nullptr;
+  if (src->device != c->device) { Error::set("vsg_seqset_revcomp: the set belongs to another device"); return VSG_EINVAL; }
+  VSG_CUDA_OK(cudaSetDevice(c->device));
+  return seqset_revcomp(c, src, q0, n, out);
+}
 
 extern "C" int64_t vsg_seqset_count(const vsg_seqset * s) { return s != nullptr ? s->d.n : 0; }
 

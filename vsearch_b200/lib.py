@@ -234,6 +234,14 @@ class Context:
                                         C.c_int64(n), C.c_int(0), C.byref(h)), "vsg_seqset_create")
         return SeqSetHandle(self, h, n, None)
 
+    def revcomp(self, ss: SeqSetHandle, q0: int = 0, n: Optional[int] = None) -> SeqSetHandle:
+        """vsg_seqset_revcomp: the reverse complements of sequences [q0, q0 + n) of ss as a new set (case kept)"""
+        n = ss.n - q0 if n is None else n
+        h = C.c_void_p()
+        _check(load().vsg_seqset_revcomp(self.h, ss.h, C.c_int64(q0), C.c_int64(n), C.byref(h)), "vsg_seqset_revcomp")
+        lens = None if ss.lens is None else np.ascontiguousarray(ss.lens[q0:q0 + n])
+        return SeqSetHandle(self, h, n, lens)
+
     def align_pairs(self, qs: SeqSetHandle, ts: SeqSetHandle, qidx: np.ndarray, tidx: np.ndarray,
                     cigar: bool = False) -> AlignResult:
         lib = load()
