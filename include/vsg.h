@@ -168,7 +168,9 @@ void vsg_index_destroy(vsg_index * ix);
  *      of `queries` in [q0, q0+nq).  For query q the best-first list (count desc, target length
  *      asc, target number asc) of at most tophits targets with count >= min(minwordmatches,
  *      number of distinct query k-mers) is written to cand_seqno/cand_count[(q-q0)*tophits ...],
- *      its length to ncand[q-q0].  Host pointers. ---- */
+ *      its length to ncand[q-q0].  Host pointers.  Any tophits >= 1: up to 1 024 one ranking pass with
+ *      the list in shared memory; beyond, two counting passes and a segmented sort (any list length,
+ *      up to the whole database). ---- */
 int vsg_rank(vsg_ctx * ctx, const vsg_index * ix, const vsg_seqset * queries, int64_t q0,
              int64_t nq, int minwordmatches, int tophits, int mask_lower,
              uint32_t * cand_seqno, uint32_t * cand_count, int32_t * ncand);
@@ -251,7 +253,9 @@ typedef struct vsg_search_result {
 void vsg_search_opts_default(vsg_search_opts * o);
 /* results[(q)*max_results + j], counts[q]; work (optional, 4 x int64): {pairs, DP cells} the
  * reference's driver hands to search16 for the same queries, then {pairs, DP cells} actually
- * aligned here (identical unless opts->lazy). */
+ * aligned here (identical unless opts->lazy).  Any maxaccepts / maxrejects (0 = all, as the command
+ * line clamps them to the database size): candidate lists longer than 1 024 are ranked in two passes
+ * and searched in pieces of bounded candidate volume. */
 int vsg_search_batch(vsg_ctx * ctx, const vsg_index * ix, const vsg_seqset * db,
                      const vsg_seqset * queries, int64_t q0, int64_t nq,
                      const vsg_search_opts * opts, vsg_search_result * results, int max_results,
@@ -373,7 +377,8 @@ int vsg_group_allpairs(vsg_group * g, const vsg_search_opts * opts, vsg_pair_hit
  *      a reader thread parses the FASTA file (headers cut at the first blank unless notrunclabels), the calling
  *      thread runs vsg_group_search on every GPU of the group (query upload, optional DUST, ranking, alignment,
  *      accept/reject, hit table download), a writer thread formats the rows of min(maxhits, hits) per query IN INPUT
- *      ORDER (the reference's order with --threads 1).  target_labels: the database headers as the reference would
+ *      ORDER (the reference's order with --threads 1); no other bound on the rows of a query (--maxaccepts 0 may
+ *      report the whole database).  target_labels: the database headers as the reference would
  *      print them.  output_no_hits != 0: the "*" row for queries without a hit.  stats (optional) receives counts and
  *      the busy seconds of each stage. ---- */
 typedef struct vsg_stream_stats {

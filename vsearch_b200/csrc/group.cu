@@ -175,11 +175,12 @@ int slice_fallback(void * u, int64_t query, int32_t strand, int64_t target, int6
 }
 }  // namespace
 
-extern "C" int vsg_group_search(vsg_group * g, const char * qcat, const int64_t * qoff, const int32_t * qlen, int64_t nq,
-                                int dust_queries, const vsg_search_opts * opts, vsg_search_result * results, int max_results,
-                                int32_t * counts, int64_t * work)
+// vsg_group_search; the rows of query q go to results[q * max_results ...] or, with rows != nullptr, to rows[q]
+static int group_search(vsg_group * g, const char * qcat, const int64_t * qoff, const int32_t * qlen, int64_t nq,
+                        int dust_queries, const vsg_search_opts * opts, vsg_search_result * results, int64_t max_results,
+                        std::vector<vsg_search_result> * rows, int32_t * counts, int64_t * work)
 {
-  if (g == nullptr || opts == nullptr || results == nullptr || counts == nullptr || nq < 0 ||
+  if (g == nullptr || opts == nullptr || counts == nullptr || nq < 0 ||
       (nq > 0 && (qcat == nullptr || qoff == nullptr || qlen == nullptr))) { Error::set("vsg_group_search: bad argument"); return VSG_EINVAL; }
   int const nd = static_cast<int>(g->ctx.size());
   if (work != nullptr) { work[0] = work[1] = work[2] = work[3] = 0; }
@@ -216,9 +217,12 @@ extern "C" int vsg_group_search(vsg_group * g, const char * qcat, const int64_t 
     vsg_search_opts o = *opts;
     if (o.query_sizes != nullptr) { o.query_sizes += b0; }
     if (o.query_labels != nullptr) { o.query_labels += b0; }
-    if (rc == VSG_OK) {
+    if (rc == VSG_OK && rows != nullptr) {
+      rc = search_batch_rows(c, g->index[static_cast<size_t>(d)], g->db[static_cast<size_t>(d)], q, 0, b1 - b0, &o,
+                             max_results, rows + b0, counts + b0, w.data() + 4 * d);
+    } else if (rc == VSG_OK) {
       rc = vsg_search_batch(c, g->index[static_cast<size_t>(d)], g->db[static_cast<size_t>(d)], q, 0, b1 - b0, &o,
-                            results + static_cast<size_t>(b0) * max_results, max_results, counts + b0, w.data() + 4 * d);
+                            results + static_cast<size_t>(b0) * max_results, static_cast<int>(max_results), counts + b0, w.data() + 4 * d);
     }
     if (rc != VSG_OK) { rcs[static_cast<size_t>(d)] = rc; msgs[static_cast<size_t>(d)] = vsg_last_error(); }
     if (g->fallback != nullptr) { vsg_ctx_set_fallback(c, g->fallback, g->fallback_user); }
@@ -235,6 +239,22 @@ extern "C" int vsg_group_search(vsg_group * g, const char * qcat, const int64_t 
     if (work != nullptr) { for (int z = 0; z < 4; z++) { work[z] += w[static_cast<size_t>(4 * d + z)]; } }
   }
   return VSG_OK;
+}
+
+extern "C" int vsg_group_search(vsg_group * g, const char * qcat, const int64_t * qoff, const int32_t * qlen, int64_t nq,
+                                int dust_queries, const vsg_search_opts * opts, vsg_search_result * results, int max_results,
+                                int32_t * counts, int64_t * work)
+{
+  if (results == nullptr) { Error::set("vsg_group_search: bad argument"); return VSG_EINVAL; }
+  return group_search(g, qcat, qoff, qlen, nq, dust_queries, opts, results, max_results, nullptr, counts, work);
+}
+
+int vsg::group_search_rows(vsg_group * g, const char * qcat, const int64_t * qoff, const int32_t * qlen, int64_t nq,
+                           int dust_queries, const vsg_search_opts * opts, int64_t max_rows, std::vector<vsg_search_result> * rows,
+                           int32_t * counts, int64_t * work)
+{
+  if (rows == nullptr) { Error::set("vsg_group_search: bad argument"); return VSG_EINVAL; }
+  return group_search(g, qcat, qoff, qlen, nq, dust_queries, opts, nullptr, max_rows, rows, counts, work);
 }
 
 extern "C" int vsg_group_allpairs(vsg_group * g, const vsg_search_opts * opts, vsg_pair_hit * hits, int64_t cap,

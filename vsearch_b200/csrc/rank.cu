@@ -277,12 +277,23 @@ __device__ __forceinline__ uint64_t make_key(uint32_t count, uint32_t len, uint3
          static_cast<uint64_t>(0xffffffu - seqno);
 }
 
-template <bool INCR>
+// What a rank_kernel launch computes per query.
+//   RANK_TOP:   the best `tophits` candidates, sorted, into out_seqno / out_count (row qi * tophits), their number to out_n.
+//   RANK_COUNT: (ranking without the TOPHITS_MAX ceiling, pass A) a histogram of the saturated counts >= minmatches over
+//               all shards, in this CTA's `hist` row; from it the threshold T (the largest count with at least tophits
+//               targets at or above it, else minmatches) to qT[qi] and the exact number K of targets >= T to out_n[qi].
+//   RANK_EMIT:  (pass B) the unsorted keys of the K targets with count >= qT[qi] to keys[key_off[qi] ...]; a count that
+//               differs from key_off[qi + 1] - key_off[qi] sets *status to 2.
+enum { RANK_TOP = 0, RANK_COUNT = 1, RANK_EMIT = 2 };
+
+template <bool INCR, int MODE = RANK_TOP>
 __global__ void __launch_bounds__(RANK_THREADS, 2)
 rank_kernel(DevSeqs qs, int64_t q0, int nq, DevSeqs db, const ShardDev * __restrict__ shards, int nshards,
             int k, int mask_lower, int minwordmatches, int tophits,
             uint32_t * __restrict__ out_seqno, uint32_t * __restrict__ out_count, int32_t * __restrict__ out_n,
-            int32_t * __restrict__ status, uint32_t * __restrict__ scratch, size_t scratch_stride, int bitmap_words, int flat)
+            int32_t * __restrict__ status, uint32_t * __restrict__ scratch, size_t scratch_stride, int bitmap_words, int flat,
+            uint32_t * __restrict__ qT = nullptr, const int32_t * __restrict__ key_off = nullptr,
+            uint64_t * __restrict__ keys = nullptr, uint32_t * __restrict__ hist_rows = nullptr, int hist_stride = 0)
 {
   extern __shared__ __align__(16) unsigned char smem[];
   uint64_t * const cand = reinterpret_cast<uint64_t *>(smem);                     // CAND_CAP
@@ -383,7 +394,15 @@ rank_kernel(DevSeqs qs, int64_t q0, int nq, DevSeqs db, const ShardDev * __restr
     // least `tophits` targets at or above it.  A target below T can never reach the final list, so
     // only counts >= T are turned into candidate keys: a few dozen per shard instead of the ~3 % of
     // all targets that pass the reference's fixed threshold (searchcore.cpp:320), no overflow sorts.
-    bool const running = !longq && (np2 + nk + 1 <= KMER_CAP);
+    bool const running = MODE == RANK_TOP && !longq && (np2 + nk + 1 <= KMER_CAP);
+    // RANK_COUNT: counts saturate at 32767 as the reference's do, so min(nk, 32767) + 1 bins (HBM: a long query's
+    // bins do not fit in shared memory)
+    int const hbins = (nk < 32767 ? nk : 32767) + 1;
+    uint32_t * const qhist = MODE == RANK_COUNT ? hist_rows + static_cast<size_t>(blockIdx.x) * hist_stride : nullptr;
+    if constexpr (MODE == RANK_COUNT) { for (int i = threadIdx.x; i < hbins; i += blockDim.x) { qhist[i] = 0; } }
+    // RANK_EMIT: T of this query and the room pass A counted for it
+    uint32_t const emit_T = MODE == RANK_EMIT ? qT[qi] : 0u;
+    int const emit_n = MODE == RANK_EMIT ? key_off[qi + 1] - key_off[qi] : 0;
     uint32_t * const hist = kmers + np2;  // nk + 1 bins in the unused tail of the k-mer array
     if (running) {
       for (int i = threadIdx.x; i <= nk; i += blockDim.x) { hist[i] = 0; }
@@ -662,6 +681,22 @@ rank_kernel(DevSeqs qs, int64_t q0, int nq, DevSeqs db, const ShardDev * __restr
 #endif
       __syncthreads();
       }  // chunk
+      if constexpr (MODE != RANK_TOP) {
+        if (MODE == RANK_COUNT || emit_n > 0) {
+          scan_counters(S.nt, MODE == RANK_COUNT ? minmatches : emit_T, VSG_RANK_ZFUSE, [&](uint32_t c, int lt) {
+            if constexpr (MODE == RANK_COUNT) {
+              atomicAdd(&qhist[c < 32767u ? c : 32767u], 1u);
+            } else {
+              int const t = S.t0 + lt;
+              int const pos = atomicAdd(&s_ncand, 1);
+              if (pos < emit_n) { keys[key_off[qi] + pos] = make_key(c, static_cast<uint32_t>(db.len[t]), static_cast<uint32_t>(t)); }
+            }
+          });
+          clean = VSG_RANK_ZFUSE != 0;
+        }
+        __syncthreads();
+        continue;  // next shard
+      }
       int const nwords = (S.nt + 1) >> 1;
       uint32_t thr = minmatches;
       if (running) {
@@ -774,6 +809,37 @@ rank_kernel(DevSeqs qs, int64_t q0, int nq, DevSeqs db, const ShardDev * __restr
         }
         __syncthreads();
       }
+    }
+    if constexpr (MODE == RANK_COUNT) {
+      // suffix sums over the bins from the top: T = the first bin where they reach tophits
+      __syncthreads();
+      if (warp == 0) {
+        int const lo = static_cast<int>(minmatches);
+        int acc = 0, T = lo, K = -1;
+        for (int top = hbins - 1; top >= lo; top -= 32) {
+          int const b = top - lane;
+          int v = b >= lo ? static_cast<int>(qhist[b]) : 0;
+#pragma unroll
+          for (int d = 1; d < 32; d <<= 1) { int const o = __shfl_up_sync(0xffffffffu, v, d); if (lane >= d) { v += o; } }
+          unsigned const hit = __ballot_sync(0xffffffffu, acc + v >= tophits);
+          if (hit != 0u) {
+            int const first = __ffs(hit) - 1;
+            T = top - first;
+            K = acc + __shfl_sync(0xffffffffu, v, first);
+            break;
+          }
+          acc += __shfl_sync(0xffffffffu, v, 31);
+        }
+        if (K < 0) { K = acc; }   // fewer than tophits targets: all of them
+        if (lane == 0) { qT[qi] = static_cast<uint32_t>(T); out_n[qi] = K; }
+      }
+      __syncthreads();
+      continue;  // next query
+    }
+    if constexpr (MODE == RANK_EMIT) {
+      if (threadIdx.x == 0 && s_ncand != emit_n) { atomicExch(status, 2); }
+      __syncthreads();
+      continue;  // next query
     }
     // 5. final order.  Usually far more targets pass the k-mer threshold than are wanted: find the
     //    count T of the tophits-th best with a histogram, keep count >= T, sort only those.
@@ -1110,17 +1176,56 @@ namespace vsg {
 const vsg_seqset * index_db(const vsg_index * ix) { return ix->db; }
 int index_wordlength(const vsg_index * ix) { return ix->k; }
 
+void rank_collect_time(vsg_ctx * c);
+
+// launch geometry of a static-index ranking and the HBM scratch of queries with more than KMER_CAP windows
+struct RankLaunch {
+  int grid = 0, maxlen = 0, bitmap_words = 1;
+  uint32_t * scratch = nullptr;
+  size_t stride = 0;
+};
+static int rank_launch_setup(vsg_ctx * c, const vsg_index * ix, const vsg_seqset * queries, int64_t q0, int64_t nq, RankLaunch & L)
+{
+  int sms = 148;
+  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, c->device);
+  L.grid = static_cast<int>(std::min<int64_t>(nq, static_cast<int64_t>(sms) * 2));
+  // queries with more than KMER_CAP windows de-duplicate their k-mers in HBM scratch
+  L.maxlen = 0;
+  for (int64_t q = q0; q < q0 + nq; q++) { L.maxlen = std::max(L.maxlen, queries->h_len[static_cast<size_t>(q)]); }
+  L.scratch = nullptr;
+  L.stride = 0;
+  L.bitmap_words = std::max(1, (1 << (2 * std::min(ix->k, 10))) >> 5);
+  if (ix->k > 10) { L.bitmap_words = 4096; while (L.bitmap_words < 2 * L.maxlen) { L.bitmap_words <<= 1; } }   // hash slots (power of two)
+  if (L.maxlen - ix->k + 1 > KMER_CAP) {
+    L.stride = static_cast<size_t>(L.bitmap_words) + static_cast<size_t>(L.maxlen) + 8;
+    int const rc = c->rank_scratch.reserve(sizeof(uint32_t) * L.stride * static_cast<size_t>(L.grid));
+    if (rc != VSG_OK) { return rc; }
+    L.scratch = static_cast<uint32_t *>(c->rank_scratch.p);
+  }
+  return VSG_OK;
+}
+static int rank_flat_mode()
+{
+  static int const rank_flat = [] { const char * e = std::getenv("VSG_RANK_FLAT"); return (e == nullptr || e[0] != '0') ? 1 : 0; }();
+  return rank_flat;
+}
+static int rank_check_args(vsg_ctx * c, const vsg_index * ix, const vsg_seqset * queries, int64_t q0, int64_t nq)
+{
+  if (q0 < 0 || nq < 0 || q0 + nq > queries->d.n) { Error::set("vsg_rank: query range out of bounds"); return VSG_EINVAL; }
+  if (queries->device != c->device || ix->device != c->device) { Error::set("vsg_rank: sequence set / index lives on another device than the context"); return VSG_EINVAL; }
+  return VSG_OK;
+}
+
 // device-side results left in ctx->rank_tmp: [seqno nq*tophits][count nq*tophits][n nq][status 1]
 int rank_enqueue(vsg_ctx * c, const vsg_index * ix, const vsg_seqset * queries, int64_t q0, int64_t nq,
                  int minwordmatches, int tophits, int mask_lower, uint32_t ** d_seqno, uint32_t ** d_count,
                  int32_t ** d_n, int32_t ** d_status)
 {
   if (tophits < 1 || tophits > TOPHITS_MAX) { Error::set("vsg_rank: tophits must be in 1..1024"); return VSG_EINVAL; }
-  if (q0 < 0 || nq < 0 || q0 + nq > queries->d.n) { Error::set("vsg_rank: query range out of bounds"); return VSG_EINVAL; }
-  if (queries->device != c->device || ix->device != c->device) { Error::set("vsg_rank: sequence set / index lives on another device than the context"); return VSG_EINVAL; }
+  int rc;
+  if ((rc = rank_check_args(c, ix, queries, q0, nq)) != VSG_OK) { return rc; }
   if (nq > (1 << 30) / tophits) { Error::set("vsg_rank: batch too large"); return VSG_EINVAL; }
   size_t const cells = static_cast<size_t>(nq) * tophits;
-  int rc;
   if ((rc = c->rank_tmp.reserve(sizeof(uint32_t) * (2 * cells + nq + 4))) != VSG_OK) { return rc; }
   *d_seqno = static_cast<uint32_t *>(c->rank_tmp.p);
   *d_count = *d_seqno + cells;
@@ -1130,30 +1235,154 @@ int rank_enqueue(vsg_ctx * c, const vsg_index * ix, const vsg_seqset * queries, 
   if (nq == 0) { return VSG_OK; }
   cudaStream_t const rs = c->stream;
   VSG_CUDA_OK(cudaFuncSetAttribute(rank_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(RANK_SMEM)));
-  int sms = 148;
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, c->device);
-  int const grid = static_cast<int>(std::min<int64_t>(nq, static_cast<int64_t>(sms) * 2));
-  // queries with more than KMER_CAP windows de-duplicate their k-mers in HBM scratch
-  int maxlen = 0;
-  for (int64_t q = q0; q < q0 + nq; q++) { maxlen = std::max(maxlen, queries->h_len[static_cast<size_t>(q)]); }
-  uint32_t * d_scratch = nullptr;
-  size_t stride = 0;
-  int bitmap_words = std::max(1, (1 << (2 * std::min(ix->k, 10))) >> 5);
-  if (ix->k > 10) { bitmap_words = 4096; while (bitmap_words < 2 * maxlen) { bitmap_words <<= 1; } }   // hash slots (power of two)
-  if (maxlen - ix->k + 1 > KMER_CAP) {
-    stride = static_cast<size_t>(bitmap_words) + static_cast<size_t>(maxlen) + 8;
-    if ((rc = c->rank_scratch.reserve(sizeof(uint32_t) * stride * static_cast<size_t>(grid))) != VSG_OK) { return rc; }
-    d_scratch = static_cast<uint32_t *>(c->rank_scratch.p);
-  }
-  static int const rank_flat = [] { const char * e = std::getenv("VSG_RANK_FLAT"); return (e == nullptr || e[0] != '0') ? 1 : 0; }();
+  RankLaunch L;
+  if ((rc = rank_launch_setup(c, ix, queries, q0, nq, L)) != VSG_OK) { return rc; }
   VSG_CUDA_OK(cudaEventRecord(c->ev[4], rs));
-  rank_kernel<false><<<grid, RANK_THREADS, RANK_SMEM, rs>>>(
+  rank_kernel<false><<<L.grid, RANK_THREADS, RANK_SMEM, rs>>>(
       queries->d, q0, static_cast<int>(nq), ix->db->d, static_cast<const ShardDev *>(ix->b_shards.p),
       static_cast<int>(ix->h_shards.size()), ix->k, mask_lower, minwordmatches, tophits, *d_seqno, *d_count, *d_n,
-      *d_status, d_scratch, stride, bitmap_words, rank_flat);
+      *d_status, L.scratch, L.stride, L.bitmap_words, rank_flat_mode());
   count_launch();
   VSG_CUDA_OK(cudaEventRecord(c->ev[5], rs));
   c->rank_pending = true;
+  return VSG_OK;
+}
+
+// ---- ranking without the TOPHITS_MAX ceiling ------------------------------------------------------------------------
+// RANK_TOP keeps its candidate keys in shared memory (CAND_CAP) and cuts them with an in-block sort, which is what makes
+// the default limits fast; longer lists (--maxaccepts 0, --maxrejects 0, large limits) are ranked in two passes over the
+// same counting code instead:
+//   rank_all_count  pass A: per query the threshold T and the exact number K of targets with count >= T (host arrays);
+//                   the caller sizes its work from K before anything large is allocated
+//   rank_all_emit   pass B: the K keys of every query of a range into one buffer, one segmented sort (descending), the
+//                   first min(K, tophits) keys of each query as CSR (seqno, count) on the device
+// Equal to search_topscores + minheap: the keys carry the heap's order, and every target with count >= T is sorted, so
+// ties at the cut are broken as the heap breaks them.
+__global__ void rank_all_gather_kernel(const uint64_t * __restrict__ keys, const int32_t * __restrict__ koff,
+                                       const int32_t * __restrict__ coff, int nq, uint32_t * __restrict__ seqno,
+                                       uint32_t * __restrict__ count)
+{
+  for (int qi = blockIdx.x; qi < nq; qi += gridDim.x) {
+    int const n = coff[qi + 1] - coff[qi];
+    const uint64_t * __restrict__ kq = keys + koff[qi];
+    for (int j = threadIdx.x; j < n; j += blockDim.x) {
+      uint64_t const key = kq[j];
+      seqno[coff[qi] + j] = 0xffffffu - static_cast<uint32_t>(key & 0xffffffu);
+      count[coff[qi] + j] = static_cast<uint32_t>(key >> 49);
+    }
+  }
+}
+
+int rank_all_count(vsg_ctx * c, const vsg_index * ix, const vsg_seqset * queries, int64_t q0, int64_t nq,
+                   int minwordmatches, int tophits, int mask_lower, uint32_t * h_T, int32_t * h_K)
+{
+  if (tophits < 1) { Error::set("vsg_rank: tophits must be at least 1"); return VSG_EINVAL; }
+  int rc;
+  if ((rc = rank_check_args(c, ix, queries, q0, nq)) != VSG_OK) { return rc; }
+  if (nq == 0) { return VSG_OK; }
+  if (nq > (1 << 28)) { Error::set("vsg_rank: batch too large"); return VSG_EINVAL; }
+  if ((rc = c->rall_q.reserve(sizeof(uint32_t) * (2 * static_cast<size_t>(nq) + 4))) != VSG_OK) { return rc; }
+  uint32_t * const d_T = static_cast<uint32_t *>(c->rall_q.p);
+  int32_t * const d_K = reinterpret_cast<int32_t *>(d_T + nq);
+  int32_t * const d_status = d_K + nq;
+  cudaStream_t const rs = c->stream;
+  VSG_CUDA_OK(cudaMemsetAsync(d_status, 0, sizeof(int32_t), rs));
+  VSG_CUDA_OK(cudaFuncSetAttribute(rank_kernel<false, RANK_COUNT>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(RANK_SMEM)));
+  RankLaunch L;
+  if ((rc = rank_launch_setup(c, ix, queries, q0, nq, L)) != VSG_OK) { return rc; }
+  int const hstride = (std::min(std::max(L.maxlen - ix->k + 1, 0), 32767) + 1 + 31) & ~31;
+  if ((rc = c->rall_hist.reserve(sizeof(uint32_t) * static_cast<size_t>(hstride) * static_cast<size_t>(L.grid))) != VSG_OK) { return rc; }
+  VSG_CUDA_OK(cudaEventRecord(c->ev[4], rs));
+  rank_kernel<false, RANK_COUNT><<<L.grid, RANK_THREADS, RANK_SMEM, rs>>>(
+      queries->d, q0, static_cast<int>(nq), ix->db->d, static_cast<const ShardDev *>(ix->b_shards.p),
+      static_cast<int>(ix->h_shards.size()), ix->k, mask_lower, minwordmatches, tophits, nullptr, nullptr, d_K,
+      d_status, L.scratch, L.stride, L.bitmap_words, rank_flat_mode(), d_T, nullptr, nullptr,
+      static_cast<uint32_t *>(c->rall_hist.p), hstride);
+  count_launch();
+  VSG_CUDA_OK(cudaEventRecord(c->ev[5], rs));
+  c->rank_pending = true;
+  int32_t status = 0;
+  VSG_CUDA_OK(cudaMemcpyAsync(h_T, d_T, sizeof(uint32_t) * static_cast<size_t>(nq), cudaMemcpyDeviceToHost, rs));
+  VSG_CUDA_OK(cudaMemcpyAsync(h_K, d_K, sizeof(int32_t) * static_cast<size_t>(nq), cudaMemcpyDeviceToHost, rs));
+  VSG_CUDA_OK(cudaMemcpyAsync(&status, d_status, sizeof(int32_t), cudaMemcpyDeviceToHost, rs));
+  VSG_CUDA_OK(cudaStreamSynchronize(rs));
+  VSG_CUDA_OK(cudaGetLastError());
+  rank_collect_time(c);
+  if (status != 0) { Error::set("vsg_rank: a query is longer than the device ranker supports (65 534 + wordlength nt)"); return VSG_EINVAL; }
+  return VSG_OK;
+}
+
+int rank_all_emit(vsg_ctx * c, const vsg_index * ix, const vsg_seqset * queries, int64_t q0, int64_t nq,
+                  int minwordmatches, int tophits, int mask_lower, const uint32_t * h_T, const int32_t * h_K,
+                  uint32_t ** d_seqno, uint32_t ** d_count, const int32_t ** d_coff)
+{
+  *d_seqno = nullptr; *d_count = nullptr; *d_coff = nullptr;
+  int rc;
+  if ((rc = rank_check_args(c, ix, queries, q0, nq)) != VSG_OK) { return rc; }
+  if (nq == 0) { return VSG_OK; }
+  // key offsets, candidate offsets, T, n, status
+  size_t const n1 = static_cast<size_t>(nq) + 1;
+  std::vector<int32_t> h(2 * n1 + 2 * static_cast<size_t>(nq) + 1, 0);
+  int64_t kt = 0, ct = 0;
+  for (int64_t i = 0; i < nq; i++) {
+    h[static_cast<size_t>(i)] = static_cast<int32_t>(kt);
+    h[n1 + static_cast<size_t>(i)] = static_cast<int32_t>(ct);
+    h[2 * n1 + static_cast<size_t>(i)] = static_cast<int32_t>(h_T[i]);
+    kt += h_K[i];
+    ct += std::min<int64_t>(h_K[i], tophits);
+    if (kt > INT32_MAX - 64) { Error::set("vsg_rank: more than 2^31 candidate keys in one call"); return VSG_EINVAL; }
+  }
+  h[static_cast<size_t>(nq)] = static_cast<int32_t>(kt);
+  h[n1 + static_cast<size_t>(nq)] = static_cast<int32_t>(ct);
+  if ((rc = c->rall_q.reserve(sizeof(int32_t) * h.size())) != VSG_OK ||
+      (rc = c->rall_keys.reserve(sizeof(uint64_t) * (2 * static_cast<size_t>(kt) + 2))) != VSG_OK ||
+      (rc = c->rall_out.reserve(sizeof(uint32_t) * (2 * static_cast<size_t>(ct) + 2))) != VSG_OK) { return rc; }
+  int32_t * const d_koff = static_cast<int32_t *>(c->rall_q.p);
+  int32_t * const d_cand_off = d_koff + n1;
+  uint32_t * const d_T = reinterpret_cast<uint32_t *>(d_cand_off + n1);
+  int32_t * const d_n = reinterpret_cast<int32_t *>(d_T + nq);
+  int32_t * const d_status = d_n + nq;
+  uint64_t * const keys0 = static_cast<uint64_t *>(c->rall_keys.p);
+  uint64_t * const keys1 = keys0 + kt + 1;
+  uint32_t * const out = static_cast<uint32_t *>(c->rall_out.p);
+  cudaStream_t const rs = c->stream;
+  // pageable source: staged before the call returns
+  VSG_CUDA_OK(cudaMemcpyAsync(d_koff, h.data(), sizeof(int32_t) * h.size(), cudaMemcpyHostToDevice, rs));
+  VSG_CUDA_OK(cudaFuncSetAttribute(rank_kernel<false, RANK_EMIT>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(RANK_SMEM)));
+  RankLaunch L;
+  if ((rc = rank_launch_setup(c, ix, queries, q0, nq, L)) != VSG_OK) { return rc; }
+  VSG_CUDA_OK(cudaEventRecord(c->ev[4], rs));
+  rank_kernel<false, RANK_EMIT><<<L.grid, RANK_THREADS, RANK_SMEM, rs>>>(
+      queries->d, q0, static_cast<int>(nq), ix->db->d, static_cast<const ShardDev *>(ix->b_shards.p),
+      static_cast<int>(ix->h_shards.size()), ix->k, mask_lower, minwordmatches, tophits, nullptr, nullptr, d_n,
+      d_status, L.scratch, L.stride, L.bitmap_words, rank_flat_mode(), d_T, d_koff, keys0, nullptr, 0);
+  count_launch();
+  if (kt > 0) {
+    size_t tb = 0;
+    VSG_CUDA_OK(cub::DeviceSegmentedSort::SortKeysDescending(nullptr, tb, keys0, keys1, static_cast<int>(kt), static_cast<int>(nq),
+                                                             d_koff, d_koff + 1, rs));
+    if ((rc = c->rall_tmp.reserve(tb + 16)) != VSG_OK) { return rc; }
+    VSG_CUDA_OK(cub::DeviceSegmentedSort::SortKeysDescending(c->rall_tmp.p, tb, keys0, keys1, static_cast<int>(kt), static_cast<int>(nq),
+                                                             d_koff, d_koff + 1, rs));
+    count_launch();
+    int sms = 148;
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, c->device);
+    rank_all_gather_kernel<<<static_cast<int>(std::min<int64_t>(nq, static_cast<int64_t>(sms) * 8)), 256, 0, rs>>>(
+        keys1, d_koff, d_cand_off, static_cast<int>(nq), out, out + ct);
+    count_launch();
+  }
+  VSG_CUDA_OK(cudaEventRecord(c->ev[5], rs));
+  c->rank_pending = true;
+  int32_t status = 0;
+  VSG_CUDA_OK(cudaMemcpyAsync(&status, d_status, sizeof(int32_t), cudaMemcpyDeviceToHost, rs));
+  VSG_CUDA_OK(cudaStreamSynchronize(rs));
+  VSG_CUDA_OK(cudaGetLastError());
+  rank_collect_time(c);
+  if (status == 1) { Error::set("vsg_rank: a query is longer than the device ranker supports (65 534 + wordlength nt)"); return VSG_EINVAL; }
+  if (status != 0) { Error::set("vsg_rank: the second ranking pass found another number of candidates than the first"); return VSG_ECUDA; }
+  *d_seqno = out;
+  *d_count = out + ct;
+  *d_coff = d_cand_off;
   return VSG_OK;
 }
 
@@ -1177,6 +1406,40 @@ extern "C" int vsg_rank(vsg_ctx * c, const vsg_index * ix, const vsg_seqset * qu
     return VSG_EINVAL;
   }
   VSG_CUDA_OK(cudaSetDevice(c->device));
+  if (tophits > TOPHITS_MAX) {
+    // the caller's dense rows, filled from the CSR of rank_all_emit a key budget at a time
+    std::vector<uint32_t> T(static_cast<size_t>(std::max<int64_t>(nq, 0)));
+    std::vector<int32_t> K(T.size());
+    int rc = rank_all_count(c, ix, queries, q0, nq, minwordmatches, tophits, mask_lower, T.data(), K.data());
+    if (rc != VSG_OK) { return rc; }
+    std::vector<uint32_t> hs, hc;
+    for (int64_t i0 = 0; i0 < nq;) {
+      int64_t i1 = i0, vol = 0;
+      while (i1 < nq && (i1 == i0 || vol + K[static_cast<size_t>(i1)] <= CAND_VOLUME_BUDGET)) { vol += K[static_cast<size_t>(i1++)]; }
+      uint32_t *d_seqno, *d_count;
+      const int32_t * d_coff;
+      if ((rc = rank_all_emit(c, ix, queries, q0 + i0, i1 - i0, minwordmatches, tophits, mask_lower, T.data() + i0, K.data() + i0,
+                              &d_seqno, &d_count, &d_coff)) != VSG_OK) { return rc; }
+      int64_t ct = 0;
+      for (int64_t i = i0; i < i1; i++) { ct += std::min<int64_t>(K[static_cast<size_t>(i)], tophits); }
+      hs.resize(static_cast<size_t>(ct)); hc.resize(static_cast<size_t>(ct));
+      if (ct > 0) {
+        VSG_CUDA_OK(cudaMemcpyAsync(hs.data(), d_seqno, sizeof(uint32_t) * static_cast<size_t>(ct), cudaMemcpyDeviceToHost, c->stream));
+        VSG_CUDA_OK(cudaMemcpyAsync(hc.data(), d_count, sizeof(uint32_t) * static_cast<size_t>(ct), cudaMemcpyDeviceToHost, c->stream));
+        VSG_CUDA_OK(cudaStreamSynchronize(c->stream));
+      }
+      size_t pos = 0;
+      for (int64_t i = i0; i < i1; i++) {
+        int const n = static_cast<int>(std::min<int64_t>(K[static_cast<size_t>(i)], tophits));
+        std::memcpy(cand_seqno + static_cast<size_t>(i) * tophits, hs.data() + pos, sizeof(uint32_t) * static_cast<size_t>(n));
+        std::memcpy(cand_count + static_cast<size_t>(i) * tophits, hc.data() + pos, sizeof(uint32_t) * static_cast<size_t>(n));
+        ncand[i] = n;
+        pos += static_cast<size_t>(n);
+      }
+      i0 = i1;
+    }
+    return VSG_OK;
+  }
   uint32_t *d_seqno, *d_count; int32_t *d_n, *d_status;
   int rc = rank_enqueue(c, ix, queries, q0, nq, minwordmatches, tophits, mask_lower, &d_seqno, &d_count, &d_n, &d_status);
   if (rc != VSG_OK) { return rc; }

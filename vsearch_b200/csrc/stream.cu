@@ -32,7 +32,7 @@ struct StreamBatch {
   std::vector<int64_t> off;
   std::vector<int32_t> len;
   std::vector<std::string> head;
-  std::vector<vsg_search_result> res;
+  std::vector<std::vector<vsg_search_result>> rows;   // of every query, at most --maxhits
   std::vector<int32_t> counts;
   bool last = false;
 };
@@ -160,10 +160,6 @@ extern "C" int vsg_usearch_stream(vsg_group * g, const char * const * target_lab
   }
   if (batch_queries < 1) { batch_queries = 65536; }
   if (maxhits <= 0) { maxhits = INT64_MAX; }
-  // rows kept per query: what can be reported (the accepted hits and the weak ones are at most maxaccepts + maxrejects)
-  int64_t const cap64 = std::min<int64_t>(maxhits, static_cast<int64_t>(opts->maxaccepts > 0 ? opts->maxaccepts : 1) +
-                                                   static_cast<int64_t>(opts->maxrejects > 0 ? opts->maxrejects : 0));
-  int const max_results = static_cast<int>(std::min<int64_t>(cap64, 1024));
   std::FILE * fin = std::fopen(query_fasta, "rb");
   if (fin == nullptr) { Error::set(std::string("vsg_usearch_stream: cannot open ") + query_fasta); return VSG_EINVAL; }
   std::FILE * fout = std::fopen(blast6out_path, "wb");
@@ -200,14 +196,14 @@ extern "C" int vsg_usearch_stream(vsg_group * g, const char * const * target_lab
       char row[256];
       size_t const nq = b->head.size();
       for (size_t q = 0; q < nq; q++) {
-        int64_t const n = std::min<int64_t>(maxhits, b->counts[q]);
+        int64_t const n = b->counts[q];
         if (n > 0) { st.matched++; }
         if (n == 0 && output_no_hits != 0) {
           out += b->head[q]; out += "\t*\t0.0\t0\t0\t0\t0\t0\t0\t0\t-1\t0\n";   // results.cpp:248-250
           st.rows++;
         }
         for (int64_t j = 0; j < n; j++) {
-          vsg_search_result const & r = b->res[q * static_cast<size_t>(max_results) + static_cast<size_t>(j)];
+          vsg_search_result const & r = b->rows[q][static_cast<size_t>(j)];
           int const qstart = r.strand != 0 ? r.query_length : 1, qend = r.strand != 0 ? 1 : r.query_length;
           out += b->head[q]; out += '\t'; out += target_labels[r.target];
           int const w = std::snprintf(row, sizeof row, "\t%.1f\t%d\t%d\t%d\t%d\t%d\t%d\t%d\t%d\t%d\n", r.id, r.internal_alignment_length,
@@ -227,10 +223,10 @@ extern "C" int vsg_usearch_stream(vsg_group * g, const char * const * target_lab
     if (b == nullptr || b->last) { break; }
     auto const t0 = std::chrono::steady_clock::now();
     int64_t const nq = static_cast<int64_t>(b->head.size());
-    b->res.resize(static_cast<size_t>(nq) * static_cast<size_t>(max_results));
+    b->rows.assign(static_cast<size_t>(nq), {});
     b->counts.assign(static_cast<size_t>(nq), 0);
-    rc = vsg_group_search(g, b->cat.data(), b->off.data(), b->len.data(), nq, qmask_dust, opts, b->res.data(), max_results,
-                          b->counts.data(), nullptr);
+    rc = group_search_rows(g, b->cat.data(), b->off.data(), b->len.data(), nq, qmask_dust, opts, maxhits, b->rows.data(),
+                           b->counts.data(), nullptr);
     st.search_s += seconds_since(t0);
     if (rc != VSG_OK) { break; }
     st.queries += nq; st.batches++;

@@ -276,7 +276,8 @@ extern "C" void vsg_ctx_destroy(vsg_ctx * c)
   if (c->stream != nullptr) { cudaStreamSynchronize(c->stream); }
   for (DevBuf * b : {&c->dir, &c->bnd, &c->he, &c->cigar_scratch, &c->cigar_dense, &c->stats,
                      &c->tasks_fast, &c->tasks_exact, &c->pairs, &c->cigar_len, &c->cigar_offs,
-                     &c->cub_tmp, &c->rank_tmp, &c->rank_scratch, &c->pre_flags, &c->ticket}) { b->release(); }
+                     &c->cub_tmp, &c->rank_tmp, &c->rank_scratch, &c->pre_flags, &c->ticket,
+                     &c->rall_q, &c->rall_hist, &c->rall_keys, &c->rall_out, &c->rall_tmp}) { b->release(); }
   for (PinBuf * b : {&c->h_tasks, &c->h_stats}) { b->release(); }
   for (auto & ev : c->ev) { if (ev != nullptr) { cudaEventDestroy(ev); } }
   for (auto & ev : c->ev_pool) { cudaEventDestroy(ev); }

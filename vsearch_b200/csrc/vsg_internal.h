@@ -100,6 +100,11 @@ struct PinBuf {
 
 void count_launch(int n = 1);
 
+// Candidate lists longer than the shared-memory ranker's 1 024 entries are ranked and searched in pieces of at most this
+// many candidate keys (summed over the queries and strands of a piece): 8 MB of keys on the device and, in
+// vsg_search_batch, about 150 MB of host hit records per worker thread.
+constexpr int64_t CAND_VOLUME_BUDGET = int64_t(1) << 20;
+
 // vsg_align_pairs with traceback on demand (align_ckpt.cuh, TbGate): leader_of[k] = index of pair k's group leader in
 // this call, or -1; threshold = 100 * --id (+ margin); skipped pairs return aligned = matches = mismatches = 0xffff
 int align_pairs_gated(vsg_ctx * c, const vsg_seqset * queries, const vsg_seqset * targets,
@@ -108,6 +113,15 @@ int align_pairs_gated(vsg_ctx * c, const vsg_seqset * queries, const vsg_seqset 
                       uint16_t * mismatches, uint16_t * gaps, int32_t * trims,
                       char * cigar_buf, int64_t cigar_cap, int64_t * cigar_off,
                       const int32_t * leader_of, double gate_threshold, int gate_iddef);
+
+// vsg_search_batch / vsg_group_search with the rows of query q (at most max_rows) in rows[q] instead of a dense
+// nq x max_results array: memory in proportion to the rows produced, whatever the limits (vsg_usearch_stream)
+int search_batch_rows(vsg_ctx * c, const vsg_index * ix, const vsg_seqset * db, const vsg_seqset * queries, int64_t q0,
+                      int64_t nq, const vsg_search_opts * opts, int64_t max_rows, std::vector<vsg_search_result> * rows,
+                      int32_t * counts, int64_t * work);
+int group_search_rows(vsg_group * g, const char * qcat, const int64_t * qoff, const int32_t * qlen, int64_t nq,
+                      int dust_queries, const vsg_search_opts * opts, int64_t max_rows, std::vector<vsg_search_result> * rows,
+                      int32_t * counts, int64_t * work);
 
 }  // namespace vsg
 
@@ -131,7 +145,8 @@ struct vsg_ctx {
   bool fast_disabled = false;  // VSG_DISABLE_FAST=1 (tests force the exact kernel)
   // scratch
   vsg::DevBuf dir, bnd, he, cigar_scratch, cigar_dense, stats, tasks_fast, tasks_exact, pairs,
-      cigar_len, cigar_offs, cub_tmp, rank_tmp, rank_scratch, pre_flags, ticket, gate;
+      cigar_len, cigar_offs, cub_tmp, rank_tmp, rank_scratch, pre_flags, ticket, gate,
+      rall_q, rall_hist, rall_keys, rall_out, rall_tmp;   // ranking without the tophits ceiling (rank.cu)
   vsg::PinBuf h_tasks, h_stats;
   size_t dir_budget = (size_t)64 << 30;
   cudaEvent_t ev[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
